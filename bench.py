@@ -2,6 +2,7 @@
 """bench.py -- HR frames/sec of the FRNet hot path at 4x BD, LR 3x134x320 -> HR 3x536x1280.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference|eager-gpu]
+                    [--dump-outputs DIR]   (writes the last timed step's outputs as DIR/*.npy)
 
 Workload (BASELINE.json configs[1]): TecoGAN 4x BD inference, synthetic 3x134x320 clips, 4 clips
 lock-stepped per GPU.  One "step" = one recurrent frame of all 4 clips on one GPU = 4 HR frames.
@@ -145,7 +146,7 @@ def synthetic_clips(n, t, seed=0):
     import torch
     import synthetic
     base = synthetic.make_clip(seed, min(t, 12), *LR)    # generate 12 frames, then ping-pong in time
-    idx = [i % (2 * len(base) - 2) for i in range(t)]
+    idx = [i % max(1, 2 * len(base) - 2) for i in range(t)]
     idx = [i if i < len(base) else 2 * len(base) - 2 - i for i in idx]
     one = base[idx]
     return torch.stack([torch.roll(one, shifts=17 * k, dims=-1) for k in range(n)])
@@ -167,8 +168,8 @@ def _host_threads(threads=None):
 
 
 def reference_net(device):
-    """The UNMODIFIED reference FRNet (baseline/_ref, installed by tools/vendor_reference.py) holding the
-    benchmark's seeded weights; None when the install is absent."""
+    """The UNMODIFIED reference FRNet (the checkout named by $TECOGAN_REFERENCE, see refimport.py) holding
+    the benchmark's seeded weights; None when it is not available."""
     import refimport
     if not refimport.available():
         return None
@@ -181,7 +182,7 @@ def reference_net(device):
 def cpu_reference_fps(steps, warmup, n=None):
     """The reference's own CPU path: FRNet.step on `n` lock-stepped clip-frames per step (default: the
     workload's clips_per_gpu, i.e. the SAME step as our arm), fp32, all host threads.  Falls back to the
-    operator-for-operator port (oracle/frnet_torchref.py) when baseline/_ref is not installed."""
+    operator-for-operator port (oracle/frnet_torchref.py) when TECOGAN_REFERENCE is not set."""
     import torch
     n = CLIPS_PER_GPU if n is None else n
     cores = _host_threads()
@@ -213,8 +214,8 @@ def run_reference(args, rank):
         return
     n = CLIPS_PER_GPU
     fps, dt, cores, kind = cpu_reference_fps(args.steps, max(args.warmup, 1))
-    src = ('unmodified reference FRNet.step from baseline/_ref (codes/models/networks/tecogan_nets.py:227-252)'
-           if kind == 'reference' else 'port oracle/frnet_torchref.py (baseline/_ref not installed)')
+    src = ('unmodified reference FRNet.step from $TECOGAN_REFERENCE (codes/models/networks/tecogan_nets.py:227-252)'
+           if kind == 'reference' else 'port oracle/frnet_torchref.py (TECOGAN_REFERENCE not set)')
     sample = (f'{args.steps} steps x {n} lock-stepped clip-frames {"x".join(map(str, LR))} -> x{SCALE} '
               f'(the same step as the GPU arm), {src}, fp32, {cores} host threads')
     line = {
@@ -230,14 +231,14 @@ def run_reference(args, rank):
 
 
 def eager_gpu_results(steps, warmup):
-    """Context comparator: the UNMODIFIED reference FRNet (baseline/_ref) on the same B200 through
+    """Context comparator: the UNMODIFIED reference FRNet ($TECOGAN_REFERENCE) on the same B200 through
     PyTorch's CUDA library kernels (cuDNN), same lock-stepped step, CUDA events: fp32, TF32 and fp16
     autocast.  Answers "what does the stock reference get on this GPU" (no B200 number is published)."""
     import torch
     dev = torch.device('cuda', torch.cuda.current_device())
     net = reference_net(dev)
     if net is None:
-        return {'unavailable': 'baseline/_ref not installed'}
+        return {'unavailable': 'TECOGAN_REFERENCE not set'}
     torch.backends.cudnn.benchmark = True                      # codes/main.py:216
     g = torch.Generator().manual_seed(0)
     n = CLIPS_PER_GPU
@@ -284,7 +285,7 @@ def run_eager_gpu(args, rank):
 # =============================================================================== training workloads
 # BASELINE.json configs[2] / [3]: TecoGAN 4x BD training (G + D + ping-pong), synthetic REDS-shape 10-frame
 # 3x64x64 LR crops, batch 32 per B200; N > 1 = DDP over NCCL (gradient all-reduce), weak scaling.
-# The loop is the REFERENCE's own (VSRGANModel.train from baseline/_ref: discriminator, VGG, losses and
+# The loop is the REFERENCE's own (VSRGANModel.train from $TECOGAN_REFERENCE: discriminator, VGG, losses and
 # optimisers stay PyTorch -- SURVEY.md section 2 puts them out of scope); the generator is this repo's
 # (forward + backward on the library's kernels) or, for the comparison arms, the reference's.
 TRAIN = dict(lr=(3, 64, 64), scale=4, t=10, batch=32, border=4,
@@ -294,7 +295,7 @@ TRAIN = dict(lr=(3, 64, 64), scale=4, t=10, batch=32, border=4,
 def train_config(model, batch, world):
     return {'workload': f'{"TecoGAN (G + ST-discriminator + VGG + ping-pong)" if model == "tecogan" else "FRVSR (generator only)"} '
                         f'4x BD training, synthetic REDS-shape {TRAIN["t"]}-frame 3x64x64 LR crops (GT 264x264 incl. the BD '
-                        f'border), reference training loop (baseline/_ref) with the generator under test; DDP/NCCL gradient '
+                        f'border), reference training loop ($TECOGAN_REFERENCE) with the generator under test; DDP/NCCL gradient '
                         f'all-reduce for N > 1 (BASELINE.json configs[2]/[3])',
             'batch_per_gpu': batch, 'global_batch': batch * world, 'frames_per_step': batch * TRAIN['t'] * world,
             'weights': 'seeded random init (no checkpoint; VGG19 = random weights of the same architecture)',
@@ -398,6 +399,10 @@ def run_train(args, rank, world, local_rank):
     model = 'frvsr' if args.workload == 'train-frvsr' else 'tecogan'
     impl = args.impl
     K, Wm = args.steps, max(args.warmup, 1)
+    import refimport
+    if not refimport.available():
+        sys.exit(f'bench.py --workload {args.workload} drives the reference\'s own training loop (VSRModel / '
+                 f'VSRGANModel, discriminator, VGG, losses): set {refimport.ENV} to the root of a TecoGAN-PyTorch checkout')
     if impl == 'reference':
         # the reference's own training step on the host cores: a bounded sample (1 clip per step)
         if rank != 0:
@@ -406,17 +411,17 @@ def run_train(args, rank, world, local_rank):
         n = 1
         m = _train_model(model, 'cpu', 'reference', False, 0, 1)
         data = torch.rand(n, TRAIN['t'], 3, 264, 264, generator=torch.Generator().manual_seed(0))
-        steps = min(K, 3)
+        steps = K
         _train_steps(m, data, 1, lambda: None)
         dt = _train_steps(m, data, steps, lambda: None)
         fps = n * TRAIN['t'] * steps / dt
         line = {'impl': 'reference', 'metric': TRAIN['metric'][model], 'value': fps, 'unit': 'frames/s', 'n_gpus': args.gpus,
-                'steps': args.steps, 'warmup': args.warmup, 'ms_per_step': 1e3 * dt / steps, 'higher_is_better': True,
+                'steps': steps, 'warmup': 1, 'ms_per_step': 1e3 * dt / steps, 'higher_is_better': True,
                 'scaling': 'weak', 'vs_baseline': None, 'dtype': 'f32', 'data': 'synthetic',
                 'config': train_config(model, args.batch or TRAIN['batch'], args.gpus),
                 'cpu_baseline': {'value': fps, 'unit': 'frames/s', 'cores': cores, 'kind': 'reference',
                                  'sample': f'{steps} training iterations of {n} clip ({TRAIN["t"]} frames, 64x64 LR) with the unmodified '
-                                           f'reference (baseline/_ref) on {cores} host threads -- a bounded sample of the batch'},
+                                           f'reference ($TECOGAN_REFERENCE) on {cores} host threads -- a bounded sample of the batch'},
                 'e2e': {'value': fps, 'unit': 'frames/s', 'h2d_bytes_per_step': 0, 'd2h_bytes_per_step': 0},
                 'gpu_launches': 0}
         print(json.dumps(line), flush=True)
@@ -618,6 +623,22 @@ def time_kernels(dev, pk):
     return out
 
 
+DUMP_U8_SAMPLES = 1 << 20
+
+
+def dump_outputs(out_dir, hr, u8):
+    """What the last timed step handed its caller: the HR frames hr_curr [n,c,H,W] (fp32, whole) and the
+    quantised frames [n,H,W,c] (uint8 -> float32, a fixed seeded sample of DUMP_U8_SAMPLES elements, with
+    their flat indices) -- together under 64 MB, so two builds can be compared output for output."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    u8 = u8.cpu().numpy().reshape(-1)
+    idx = np.sort(np.random.default_rng(0).choice(u8.size, size=min(DUMP_U8_SAMPLES, u8.size), replace=False))
+    np.save(os.path.join(out_dir, 'hr_curr.npy'), hr.cpu().numpy().astype(np.float32))
+    np.save(os.path.join(out_dir, 'hr_u8_sample.npy'), u8[idx].astype(np.float32))
+    np.save(os.path.join(out_dir, 'hr_u8_sample_index.npy'), idx.astype(np.float64))
+
+
 def run_ours(args, rank, world, local_rank):
     import torch
     import torch.distributed as dist
@@ -675,6 +696,9 @@ def run_ours(args, rank, world, local_rank):
     value = world * n * K / (ms_max * 1e-3)
     launches_per_step = eng.launches_per_step + 0               # kernels inside one graph replay
     gpu_launches = launches_per_step * K
+    if args.dump_outputs and rank == 0:
+        p_last = (Wm + K - 1) & 1
+        dump_outputs(args.dump_outputs, eng.hr[p_last], eng.u8[p_last])
 
     if args.profile_only:          # under ncu: only the step loop, no JSON line
         if rank == 0:
@@ -707,7 +731,7 @@ def run_ours(args, rank, world, local_rank):
                          'how': 'same device-resident step loop as `value`, run for >= %.0f s' % args.sustain_s}
 
     # ---------------- end to end through FRNet.infer_sequence with host buffers
-    t_e2e = max(K, 4) if WL_KEY == 'bd4' else 30           # config 5 is quoted on 30-frame clips
+    t_e2e = K if WL_KEY == 'bd4' else 30                   # config 5 is quoted on 30-frame clips
     host_clips = synthetic_clips(n, t_e2e, seed=100 + rank).pin_memory()     # [n,T,c,h,w] pinned
     net.infer_sequence(host_clips[:, :4], dev)                                # warm-up
     net.infer_sequence(host_clips, dev)
@@ -737,7 +761,7 @@ def run_ours(args, rank, world, local_rank):
             fps, dt, cores, kind = cpu_reference_fps(steps_cpu, 1)
             cpu = {'value': fps, 'unit': 'frames/s', 'cores': cores, 'kind': kind,
                    'sample': f'{steps_cpu} steps x {n} lock-stepped clip-frames {"x".join(map(str, LR))} (fp32, '
-                             + ('unmodified reference FRNet.step from baseline/_ref' if kind == 'reference' else
+                             + ('unmodified reference FRNet.step from $TECOGAN_REFERENCE' if kind == 'reference' else
                                 'port oracle/frnet_torchref.py') + f'), {dt:.1f} s of CPU work'}
             if not args.no_eager:
                 eager = eager_gpu_results(10, 3)
@@ -778,7 +802,9 @@ def run_ours(args, rank, world, local_rank):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=50)
+    ap.add_argument('--steps', type=int, default=50,
+                    help='timed steps (recurrent frames of the lock-stepped clips, or training iterations); also the '
+                         'frames of the e2e clip for bd4 -- bi2\'s e2e block always runs its 30-frame clips (config 5)')
     ap.add_argument('--warmup', type=int, default=5)
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference', 'eager-gpu'])
     ap.add_argument('--workload', default='bd4', choices=sorted(WORKLOADS) + ['train', 'train-frvsr'],
@@ -789,7 +815,14 @@ def main():
     ap.add_argument('--no-eager', action='store_true', help='skip the gpu_eager_baseline block (N=1 only)')
     ap.add_argument('--profile-only', action='store_true',
                     help='run only the device-resident step loop (for ncu captures); prints nothing')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write the outputs of the last timed step as DIR/<name>.npy '
+                         '(inference workloads of --impl ours; rank 0)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.impl != 'ours' or args.workload.startswith('train')):
+        ap.error('--dump-outputs writes the outputs of the timed inference step: --impl ours, --workload bd4 or bi2')
     rank = int(os.environ.get('RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))

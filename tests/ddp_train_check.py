@@ -4,13 +4,12 @@ DDP with world size 1 in `reference_training_integration_ddp`):
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29541 \
         tests/ddp_train_check.py
 
-Each rank builds the reference's VSRModel (baseline/_ref, FRVSR train.yml, dist=True -> DistributedDataParallel
-exactly as base_model.model_to_device wraps it) around tecogan_b200's generator, feeds DIFFERENT clips, runs one
-train() step, and the ranks then verify that (a) every parameter gradient is finite and identical on both ranks
-(NCCL all-reduce happened on gradients our backward kernels produced), (b) it equals the mean of the two
-single-rank gradients computed without DDP on the same clips, (c) the updated weights agree across ranks.
+Each rank runs one iteration of the reference's FRVSR training loop (gpu_checks.frvsr_train_step, nb=2) around
+tecogan_b200's generator wrapped in DistributedDataParallel as base_model.model_to_device wraps it, on DIFFERENT
+clips; the ranks then verify that (a) every parameter gradient is finite and identical on both ranks (NCCL
+all-reduce happened on gradients our backward kernels produced), (b) it equals the mean of the two single-rank
+gradients computed without DDP on the same clips, (c) the updated weights agree across ranks.
 """
-import copy
 import os
 import sys
 
@@ -18,8 +17,7 @@ import numpy as np
 import torch
 import torch.distributed as dist
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 
 
 def main():
@@ -27,7 +25,7 @@ def main():
     torch.cuda.set_device(local)
     dev = f'cuda:{local}'
     dist.init_process_group('nccl', device_id=torch.device(dev))
-    import refimport
+    import gpu_checks
     import synthetic
     import tecogan_b200 as T
     p = synthetic.make_frnet_params(41, nb=2, gain=1.5)
@@ -35,14 +33,11 @@ def main():
              for r in range(world)]
 
     def run(use_ddp, data):
-        opt = refimport.training_opt('frvsr', device=dev, dist=use_ddp, rank=rank, world_size=world, nb=2)
-        m = refimport.build_training_model(opt, T.define_generator)
-        m.get_bare_model(m.net_G).load_state_dict(p, strict=True)
-        m.prepare_training_data({'gt': data.clone()})
-        m.train()
-        net = m.get_bare_model(m.net_G)
+        net = T.FRNet(3, 3, 64, 2, 'BD', 4).to(dev)
+        net.load_state_dict(p, strict=True)
+        log = gpu_checks.frvsr_train_step(gpu_checks.ddp_wrap(net) if use_ddp else net, data.to(dev))
         return ({k: v.grad.detach().clone() for k, v in net.named_parameters()},
-                {k: v.detach().clone() for k, v in net.named_parameters()}, dict(m.log_dict))
+                {k: v.detach().clone() for k, v in net.named_parameters()}, log)
 
     g_ddp, w_ddp, log = run(True, clips[rank])
     singles = [run(False, clips[r])[0] for r in range(world)]

@@ -1,13 +1,10 @@
 """CPU: pin the oracle (oracle/) against outputs of the UNMODIFIED reference.
 
 The fixtures in tests/golden were written by oracle/gen_golden.py, which imports
-/root/reference and runs it on seeded inputs.  When /root/reference is present
-(build container) the oracle is additionally compared with the live reference at
-the BASELINE size 3x134x320.
+the reference and runs it on seeded inputs, including one step at the BASELINE
+size 3x134x320 (stored as a strided sample).
 """
 import os
-import sys
-import types
 
 import numpy as np
 import pytest
@@ -149,25 +146,18 @@ def test_state_dict_layout_matches_reference_counts():
     assert n == 2589093
 
 
-# ------------------------------------------------------------------ live reference (build container only)
-@pytest.mark.skipif(not os.path.isdir('/root/reference/codes'), reason='reference not mounted')
+# ------------------------------------------------------------------ benchmark size
 def test_oracle_vs_live_reference_full_size():
-    R = '/root/reference/codes'
-    if R not in sys.path:
-        sys.path.insert(0, R)
-    m = types.ModuleType('metrics')
-    m.__path__ = [R + '/metrics']
-    sys.modules.setdefault('metrics', m)
-    from models.networks.tecogan_nets import FRNet
-    net = FRNet(3, 3, 64, 10, 'BD', 4)
+    """FRNet.step at 3x134x320 -> 3x536x1280 against the reference's output (every 241st element and the
+    largest magnitude of the whole frame, oracle/gen_golden.py)."""
+    g = np.load(os.path.join(G, 'step_bd4_134x320_g2_sample.npz'))
     p = O.make_frnet_params(5, gain=2.0)
-    net.load_state_dict(p, strict=True)
-    net.eval()
     lr_curr, lr_prev, hr_prev = rand(1, 1, 3, 134, 320), rand(2, 1, 3, 134, 320), rand(3, 1, 3, 536, 1280)
-    with torch.no_grad():
-        ref = net.step(lr_curr, lr_prev, hr_prev)
-    hr = O.frnet_step(p, lr_curr, lr_prev, hr_prev, 4, 'BD')
-    assert relerr(hr.numpy(), ref.numpy()) <= 5e-5
+    hr = O.frnet_step(p, lr_curr, lr_prev, hr_prev, 4, 'BD').numpy()
+    assert hr.shape == tuple(g['shape'])
+    err = np.abs(hr.reshape(-1)[::241].astype(np.float64) - g['hr_sample']).max() / float(g['hr_absmax'])
+    assert err <= 5e-5
+    assert abs(float(np.abs(hr).max()) - float(g['hr_absmax'])) <= 5e-5 * float(g['hr_absmax'])
 
 
 # ------------------------------------------------------------------ library-op restatement (bench CPU baseline)
