@@ -1224,6 +1224,508 @@ def check_fused_tail(scale=4, n=2, h=20, w=26, with_lr=True, seed=400, accumulat
     return out
 
 
+# =============================================================================== backward kernels at training shapes
+# The unit checks above give every persistent CTA of the backward kernels at most one 16x8 tile.  The checks
+# below run them at the shapes of training (10 residual blocks, 19-frame ping-pong clips, 64x64 LR crops), where
+# a CTA walks many tiles: the smem stage ring wraps, the phase bit flips, later tiles accumulate onto earlier
+# ones, and the fused bias gradient reads its ones block from every stage.  The references are exact: every
+# product of two fp16 values is exact in fp64, so a float64 reference on the very fp16 operands handed to the
+# kernel leaves only the kernel's fp32 summation error, and one dropped or doubled tile out of T moves the
+# result by ~1/sqrt(T) -- orders of magnitude above the bars.
+
+WG_STAGES_SMEM = 232448          # tg_wgrad_tcgen05: dynamic smem per CTA
+
+
+def _wgrad_plan(kind, cin, cout, n, h, w, max_ctas=0, with_db=False, sms=148):
+    """Tile count, CTAs per (ci chunk, co chunk) pair, tiles per CTA and smem stage count, as tg_wgrad_tcgen05
+    computes them on the host (cin / cout = stored channel counts)."""
+    tiles = -(-w // 8) * -(-h // 16) * n
+    pairs = (cin // 64) * (cout // 64)
+    budget = max_ctas if 0 < max_ctas < sms else sms
+    budget = max(budget, pairs)
+    cpp = min(budget // pairs, tiles)
+    conv = kind == L.CONV_3X3
+    box_w, box_h = (10, 18) if conv else (9, 17)
+    stage = (box_w * box_h * 128 + 1023) // 1024 * 1024 + (1 if conv else 4) * 16384
+    ones = 3072 if (conv and with_db) else 0
+    stages = min((WG_STAGES_SMEM - 2048 - ones) // stage, 6)
+    return {'tiles': tiles, 'pairs': pairs, 'ctas_per_pair': cpp, 'tiles_per_cta': tiles / cpp,
+            'max_tiles_per_cta': -(-tiles // cpp), 'stages': stages}
+
+
+def _dgrad_plan(cout, n, h, w, max_ctas=0, sms=148):
+    """Tiles per CTA of tg_conv_tcgen05 for a data gradient (h, w = the size of dx, cout = its stored channels):
+    output channels above 64 split the tiles over cout/64 CTA groups."""
+    n_split = cout // 64 if cout > 64 else 1
+    tiles = -(-w // 8) * -(-h // 16) * n * n_split
+    grid = max_ctas if max_ctas > 0 else sms
+    grid = min(grid, tiles)
+    grid -= grid % n_split
+    grid = max(grid, n_split)
+    return {'tiles': tiles, 'grid': grid, 'tiles_per_cta': tiles / grid, 'max_tiles_per_cta': -(-tiles // grid)}
+
+
+def _host_scale(amax, target=256.0):
+    """2^clamp(floor(log2(target / amax)), -24, 24): the loss scale scale_from_amax_kernel picks"""
+    e = int(np.floor(np.log2(target / amax)))
+    return float(2.0 ** max(-24, min(24, e)))
+
+
+def _conv_bwd64(g, x, w, kind, weight_grad):
+    """d/dW (weight_grad) or d/dx of conv3x3 (pad 1) / convT3x3s2 (pad 1, output_padding 1) in float64 for the output
+    gradient g, through the kernel torch autograd runs (aten.convolution_backward); only the shapes of the
+    operand not differentiated against are used."""
+    conv = kind == L.CONV_3X3
+    st = [1, 1] if conv else [2, 2]
+    op = [0, 0] if conv else [1, 1]
+    mask = [False, True, False] if weight_grad else [True, False, False]
+    r = torch.ops.aten.convolution_backward(g, x, w, None, st, [1, 1], [1, 1], not conv, op, 1, mask)
+    return r[1] if weight_grad else r[0]
+
+
+def _wgrad_ref64(x16, dz16, kind, inv_scale, chunk=4):
+    """dW, db (float64) of a conv3x3 / convT3x3s2 layer from the fp16 operands handed to the kernel: x16 = its
+    input [n,cin_real,h,w], dz16 = the loss-scaled gradient of its output [n,cout_real,oh,ow]; times 1/scale."""
+    n, ci = x16.shape[:2]
+    co = dz16.shape[1]
+    wshape = (co, ci, 3, 3) if kind == L.CONV_3X3 else (ci, co, 3, 3)
+    dw = torch.zeros(wshape, dtype=torch.float64)
+    with torch.no_grad():
+        for i in range(0, n, chunk):                       # chunks bound the im2col buffers
+            dw += _conv_bwd64(dz16[i:i + chunk].double(), x16[i:i + chunk].double(), dw, kind, True)
+        db = dz16.double().sum((0, 2, 3))
+    return dw * inv_scale, db * inv_scale
+
+
+def _dact64(mask16, mask_act):
+    slope = 0.0 if mask_act == L.ACT_RELU else 0.2
+    m = mask16.double()
+    return torch.where(m > 0, torch.ones_like(m), torch.full_like(m, slope))
+
+
+def _dgrad_ref64(dz16, w, kind, residual16=None, mask16=None, mask_act=None, chunk=4):
+    """float64 data gradient of a conv layer, (d/dx [+ residual]) * act'(mask), from the fp16 operands handed to
+    the kernel: dz16 [n,cout_real,oh,ow], w = the layer weight (the kernel packs it as fp16), residual16 /
+    mask16 [n,cin_real,h,w]."""
+    w64 = f16(w).double()
+    up = 1 if kind == L.CONV_3X3 else 2
+    n, _, oh, ow = dz16.shape
+    cin = w.shape[1] if kind == L.CONV_3X3 else w.shape[0]
+    with torch.no_grad():
+        y = torch.cat([_conv_bwd64(dz16[i:i + chunk].double(),
+                                   torch.empty(min(chunk, n - i), cin, oh // up, ow // up, dtype=torch.float64),
+                                   w64, kind, False) for i in range(0, n, chunk)])
+        if residual16 is not None:
+            y = y + residual16.double()
+        if mask16 is not None:
+            y = y * _dact64(mask16, mask_act)
+    return y
+
+
+def _tile_mask(shape, img, ty, tx, up):
+    """[n,1,oh,ow] float64 mask of one 16x8 pixel tile of image img (up = 2: the tile seen at the convT output)"""
+    m = torch.zeros(shape[0], 1, shape[2], shape[3], dtype=torch.float64)
+    m[img, :, up * 16 * ty:up * 16 * (ty + 1), up * 8 * tx:up * 8 * (tx + 1)] = 1.0
+    return m
+
+
+def _dgrad_metric(got, ref):
+    """max over elements of |got - ref| / (1 fp16 ulp(|ref|) + 1e-5 max|ref|): <= 1 is the bar"""
+    got = np.asarray(got, np.float64)
+    ref = np.asarray(ref, np.float64)
+    ulp = np.spacing(np.abs(ref).astype(np.float16)).astype(np.float64)
+    tol = ulp + 1e-5 * np.abs(ref).max()
+    return float((np.abs(got - ref) / tol).max())
+
+
+# wgrad cases: (kind, cin_real, cout_real, n, h, w) with h, w = the layer INPUT size; runs = max_ctas values
+WGRAD_CASES = {
+    # SRNet residual conv over 2 clips x 19 frames of 64x64: ~8 tiles per CTA, the 5-stage ring wraps
+    'srnet_conv': dict(kind=L.CONV_3X3, cin_real=64, cout_real=64, n=38, h=64, w=64, runs=(0,), seed=600),
+    # conv_out 64->3 over 38 HR frames of 256x256: ~131 tiles per CTA
+    'conv_out': dict(kind=L.CONV_3X3, cin_real=64, cout_real=3, n=38, h=256, w=256, runs=(0,), seed=610),
+    # the two transposed convs (dz at 2x): the 2-stage ring wraps many times
+    'convT_64': dict(kind=L.CONVT_3X3_S2, cin_real=64, cout_real=64, n=38, h=64, w=64, runs=(0,), seed=620),
+    'convT_128': dict(kind=L.CONVT_3X3_S2, cin_real=64, cout_real=64, n=38, h=128, w=128, runs=(0,), seed=630),
+    # FNet on 36 frame pairs at LR 64x64; 2-4 tiles per CTA on the default grid, many at max_ctas=8
+    'fnet_enc1_0': dict(kind=L.CONV_3X3, cin_real=6, cout_real=32, n=36, h=64, w=64, runs=(0, 8), seed=640),
+    'fnet_dec1_0': dict(kind=L.CONV_3X3, cin_real=128, cout_real=256, n=36, h=8, w=8, runs=(0, 8), seed=650),
+    'fnet_dec1_2': dict(kind=L.CONV_3X3, cin_real=256, cout_real=256, n=36, h=8, w=8, runs=(0, 8), seed=660),
+    'fnet_dec2_0': dict(kind=L.CONV_3X3, cin_real=256, cout_real=128, n=36, h=16, w=16, runs=(0, 8), seed=670),
+    'fnet_flow_2': dict(kind=L.CONV_3X3, cin_real=32, cout_real=2, n=36, h=64, w=64, runs=(0, 8), seed=680),
+    # ragged 37x29, few CTAs: the ring wraps cheaply and the bias descriptor visits every stage index
+    'max_ctas_sweep': dict(kind=L.CONV_3X3, cin_real=64, cout_real=64, n=5, h=37, w=29, runs=(1, 2, 3, 5, 7), seed=690),
+}
+
+WG_BAR_L2, WG_BAR_MAX, WG_BAR_DB = 1e-4, 1e-3, 1e-4
+
+
+def wgrad_case_operands(case):
+    """Host operands of a wgrad case: x16 [n,cin_real,h,w] fp16, the fp32 gradient gy of the layer output (tiny,
+    like a mean-reduced loss: amax ~1e-8, so the 2^24 cap of the loss scale is active), the scale the device will
+    pick, and dz16 = fp16(gy * scale) as grad_pack stores it."""
+    c = WGRAD_CASES[case]
+    up = 1 if c['kind'] == L.CONV_3X3 else 2
+    x16 = rand(c['seed'], c['n'], c['cin_real'], c['h'], c['w'], lo=-1, hi=1).half()
+    gy = rand(c['seed'] + 1, c['n'], c['cout_real'], up * c['h'], up * c['w'], lo=-1e-8, hi=1e-8)
+    scale = _host_scale(float(gy.abs().max()))
+    return x16, gy, scale, (gy * scale).half()
+
+
+def wgrad_detection_power(case, x16=None, dz16=None, scale=None, ref=None):
+    """rel-L2 of the exact reference with the contribution of one 16x8 tile (the last tile of the last image)
+    removed, against the full reference: what a kernel that dropped that tile would score, for dW and db."""
+    c = WGRAD_CASES[case]
+    if x16 is None:
+        x16, _, scale, dz16 = wgrad_case_operands(case)
+    if ref is None:
+        ref = _wgrad_ref64(x16, dz16, c['kind'], 1.0 / scale)
+    up = 1 if c['kind'] == L.CONV_3X3 else 2
+    n = c['n']
+    m = _tile_mask(dz16.shape, 0, -(-c['h'] // 16) - 1, -(-c['w'] // 8) - 1, up)[:1]
+    part = _wgrad_ref64(x16[n - 1:n], (dz16[n - 1:n].double() * m).half(), c['kind'], 1.0 / scale)
+    return {'dw_rel_l2': rell2((ref[0] - part[0]).numpy(), ref[0].numpy()),
+            'db_rel_l2': rell2((ref[1] - part[1]).numpy(), ref[1].numpy())}
+
+
+def check_wgrad_multitile(case):
+    """tg_wgrad_tcgen05 at a training shape against the exact float64 reference (_wgrad_ref64) on the operands
+    handed to the kernel: the scale the device chose and the dz grad_pack stored are first checked to be the
+    host's, bit for bit.  dw / db are pre-filled (the kernel accumulates).  Bars: dW rel-L2 <= 1e-4 and
+    per-element |err| <= 1e-3 max|ref|, fused db rel-L2 <= 1e-4 (fp32 accumulation of exact fp16 products: the
+    only error is the fp32 summation; measured on a B200, 1.5e-6 at 8 tiles per CTA and 2.2e-5 at 144, as the
+    running sums of a CTA grow).  The CUDA-core kernel is reported as a second opinion."""
+    c = WGRAD_CASES[case]
+    kind, n, h, w = c['kind'], c['n'], c['h'], c['w']
+    up = 1 if kind == L.CONV_3X3 else 2
+    x16, gy, scale, dz16 = wgrad_case_operands(case)
+    ref_dw, ref_db = ref = _wgrad_ref64(x16, dz16, kind, 1.0 / scale)
+    det = wgrad_detection_power(case, x16, dz16, scale, ref)
+    out = {'detect_drop_tile_dw': det['dw_rel_l2'], 'detect_drop_tile_db': det['db_rel_l2'], 'scale_log2': float(np.log2(scale))}
+    assert det['dw_rel_l2'] > 10 * WG_BAR_L2 and det['db_rel_l2'] > 10 * WG_BAR_DB, out
+    wshape = tuple(ref_dw.shape)
+    fwd = ops.PackedConv(torch.zeros(wshape, device=DEV), torch.zeros(c['cout_real'], device=DEV), kind, L.ACT_NONE)
+    cpad = ops.pad64(c['cout_real'])
+    sc = ops.GradScale(DEV).from_amax(gy.to(DEV))
+    dzs = ops.grad_pack(gy.to(DEV), scale=sc, cpad=cpad)
+    xg = nhwc(x16.float(), fwd.cin)
+    torch.cuda.synchronize()
+    assert float(sc.ws[0]) == scale and float(sc.ws[1]) == 1.0 / scale, (float(sc.ws[0]), scale)
+    host_dz = torch.zeros(n, up * h, up * w, cpad, dtype=torch.float16)
+    host_dz[..., :c['cout_real']] = dz16.permute(0, 2, 3, 1)
+    assert torch.equal(dzs.cpu(), host_dz), 'grad_pack output differs from fp16(g * scale)'
+    del host_dz
+    rmax = float(ref_dw.abs().max())
+    pre_dw = rand(c['seed'] + 2, *wshape, lo=-1, hi=1) * rmax
+    pre_db = rand(c['seed'] + 3, c['cout_real'], lo=-1, hi=1) * float(ref_db.abs().max())
+    first = None
+    for mc in c['runs']:
+        plan = _wgrad_plan(kind, fwd.cin, cpad, n, h, w, mc, with_db=kind == L.CONV_3X3, sms=ops.sm_count())
+        dw, db = pre_dw.to(DEV), pre_db.to(DEV)
+        ops.wgrad(fwd, xg, dzs, dw, scale=sc, db=db, max_ctas=mc)
+        torch.cuda.synchronize()
+        got_dw = dw.cpu().double() - pre_dw.double()
+        got_db = db.cpu().double() - pre_db.double()
+        r = {'tiles_per_cta': round(plan['tiles_per_cta'], 2), 'stages': plan['stages'],
+             'dw_rel_l2': rell2(got_dw.numpy(), ref_dw.numpy()),
+             'dw_rel_max': float((got_dw - ref_dw).abs().max()) / rmax,
+             'db_rel_l2': rell2(got_db.numpy(), ref_db.numpy())}
+        if first is None:
+            first = (got_dw, got_db)
+        elif case == 'max_ctas_sweep':   # grids of 2..7 CTAs: only the order of the fp32 sums and atomics differs
+            r['vs_first_run_rel_l2'] = max(rell2(got_dw.numpy(), first[0].numpy()), rell2(got_db.numpy(), first[1].numpy()))
+            assert r['vs_first_run_rel_l2'] <= 1e-5, (case, mc, r)
+        out[f'max_ctas{mc}'] = r
+        assert r['dw_rel_l2'] <= WG_BAR_L2 and r['dw_rel_max'] <= WG_BAR_MAX and r['db_rel_l2'] <= WG_BAR_DB, (case, mc, r)
+        if case == 'max_ctas_sweep':
+            assert plan['ctas_per_pair'] == mc, (case, mc, plan)
+        if mc == 0 and case.startswith('fnet_'):
+            assert plan['tiles_per_cta'] >= 2, (case, mc, plan)                 # FNet's few tiles on the default grid
+        else:
+            assert plan['tiles_per_cta'] > plan['stages'], (case, mc, plan)     # the ring wraps on every CTA
+    # the CUDA-core kernel on the same operands (reported)
+    dw = torch.zeros(wshape, device=DEV)
+    ops.wgrad(fwd, xg, dzs, dw, scale=sc, impl='simt')
+    torch.cuda.synchronize()
+    out['simt_dw_rel_l2'] = rell2(dw.cpu().numpy(), ref_dw.numpy())
+    return out
+
+
+# dgrad cases: the forward layer (kind, cin_real, cout_real), n images of h x w (= the size of dx), the
+# derivative mask, a residual; every case runs on the default grid and on the few CTAs of `runs`
+DGRAD_CASES = {
+    # SRNet residual conv, halo BWD instance with ReLU' mask and the skip gradient
+    'srnet_halo': dict(kind=L.CONV_3X3, cin_real=64, cout_real=64, n=8, h=64, w=64, act=L.ACT_RELU, residual=True,
+                       runs=(0, 3), seed=700),
+    # conv_out: dz has 3 real channels (k-step skip), ReLU' of the last transposed conv; ~28 tiles per CTA
+    'conv_out': dict(kind=L.CONV_3X3, cin_real=64, cout_real=3, n=8, h=256, w=256, act=L.ACT_RELU, residual=False,
+                     runs=(0, 7), seed=710),
+    # transposed convs: a stride-2 conv over dz (CONV_3X3_S2, tap mode)
+    'convT_256_to_128': dict(kind=L.CONVT_3X3_S2, cin_real=64, cout_real=64, n=8, h=128, w=128, act=L.ACT_RELU,
+                             residual=False, runs=(0, 5), seed=720),
+    'convT_128_to_64': dict(kind=L.CONVT_3X3_S2, cin_real=64, cout_real=64, n=8, h=64, w=64, act=L.ACT_RELU,
+                            residual=False, runs=(0, 3), seed=730),
+    # FNet decoder2.0 256->128 at 16x16: dx has 256 channels = 4 CTA groups
+    'fnet_dec2_0': dict(kind=L.CONV_3X3, cin_real=256, cout_real=128, n=36, h=16, w=16, act=L.ACT_LRELU02,
+                        residual=False, runs=(0, 2), seed=740),
+}
+
+
+def dgrad_case_operands(case):
+    """weight [fp32, the layer's layout], dz16 [n,cout_real,oh,ow], residual16 / mask16 [n,cin_real,h,w] (fp16)"""
+    c = DGRAD_CASES[case]
+    up = 1 if c['kind'] == L.CONV_3X3 else 2
+    n, ci, co, h, w, s = c['n'], c['cin_real'], c['cout_real'], c['h'], c['w'], c['seed']
+    wshape = (co, ci, 3, 3) if c['kind'] == L.CONV_3X3 else (ci, co, 3, 3)
+    wt = rand(s, *wshape, lo=-0.1, hi=0.1)
+    dz16 = rand(s + 1, n, co, up * h, up * w, lo=-1, hi=1).half()
+    res16 = rand(s + 2, n, ci, h, w, lo=-1, hi=1).half() if c['residual'] else None
+    mask16 = rand(s + 3, n, ci, h, w, lo=-1, hi=1).half()
+    return wt, dz16, res16, mask16
+
+
+def dgrad_detection_power(case, ref=None):
+    """the per-element metric of the exact reference with one output tile (the last tile of the last image)
+    zeroed, against the full reference: what a kernel that skipped that tile would score"""
+    c = DGRAD_CASES[case]
+    if ref is None:
+        wt, dz16, res16, mask16 = dgrad_case_operands(case)
+        ref = _dgrad_ref64(dz16, wt, c['kind'], res16, mask16, c['act'])
+    m = 1.0 - _tile_mask(ref.shape, ref.shape[0] - 1, -(-c['h'] // 16) - 1, -(-c['w'] // 8) - 1, 1)
+    return _dgrad_metric((ref * m).numpy(), ref.numpy())
+
+
+def check_dgrad_multitile(case):
+    """PackedDgrad (the BWD instances of tg_conv_tcgen05 with the DRELU / DLRELU mask epilogue) at a training shape
+    against the exact float64 reference (_dgrad_ref64).  The output is poisoned with NaN first, so every element
+    must be written.  Per-element bar: |got - ref| <= 1 fp16 ulp(|ref|) + 1e-5 max|ref| -- the output is rounded
+    to fp16, nothing looser is justified.  A tile is computed by one CTA with the same MMAs in the same order
+    whichever CTA it is, so the runs on different grids must agree bit for bit."""
+    c = DGRAD_CASES[case]
+    kind = c['kind']
+    wt, dz16, res16, mask16 = dgrad_case_operands(case)
+    ref = _dgrad_ref64(dz16, wt, kind, res16, mask16, c['act'])
+    out = {'detect_zero_tile': dgrad_detection_power(case, ref)}
+    assert out['detect_zero_tile'] > 10, out
+    epi = L.EPI_OUT_NCHW_F32 if c['cout_real'] <= 3 else L.EPI_NHWC_F16        # conv_out is a thin NCHW head
+    fwd = ops.PackedConv(wt.to(DEV), torch.zeros(c['cout_real'], device=DEV), kind, L.ACT_NONE, epi)
+    dg = ops.PackedDgrad(fwd, wt.to(DEV))
+    n, h, w = c['n'], c['h'], c['w']
+    dzg = nhwc(dz16.float(), dg.cin)
+    res = nhwc(res16.float(), dg.cout) if res16 is not None else None
+    msk = nhwc(mask16.float(), dg.cout)
+    ci = c['cin_real']
+    first = None
+    for mc in c['runs']:
+        plan = _dgrad_plan(dg.cout, n, h, w, mc, sms=ops.sm_count())
+        y = torch.full((n, h, w, dg.cout), float('nan'), dtype=torch.float16, device=DEV)
+        dg(dzg, y=y, residual=res, mask=msk, mask_act=c['act'], max_ctas=mc)
+        torch.cuda.synchronize()
+        assert not bool(torch.isnan(y).any()), f'{case} max_ctas={mc}: dgrad left output elements unwritten'
+        if dg.cout > ci:
+            assert float(y[..., ci:].abs().max()) == 0.0, 'pad channels of dx must be zero'
+        got = from_nhwc(y, ci).double()
+        r = {'tiles_per_cta': round(plan['tiles_per_cta'], 2), 'ulp_metric': _dgrad_metric(got.numpy(), ref.numpy()),
+             'rel_l2': rell2(got.numpy(), ref.numpy())}
+        out[f'max_ctas{mc}'] = r
+        assert r['ulp_metric'] <= 1.0, (case, mc, r)
+        assert mc == 0 or plan['tiles_per_cta'] > 6, (case, mc, plan)          # many tiles per CTA
+        if first is None:
+            first = y
+        else:
+            assert torch.equal(y, first), f'{case}: max_ctas={mc} differs from the default grid'
+    return out
+
+
+# =============================================================================== elementwise backward past one grid pass
+GRID_STRIDE_ITEMS = 148 * 32 * 256         # items one pass of the backward kernels' capped grid-stride loop covers
+
+
+def check_backward_elementwise_large():
+    """The grid-stride elementwise backward kernels at sizes above one pass of their capped grid (148*32 blocks x 256
+    threads), with the decisive values at the LAST indices, against float64 / exact host references."""
+    out = {}
+    # ---- loss scale: amax over 38x3x256x256 with the largest |value| last; exact power of two
+    shape = (38, 3, 256, 256)
+    assert int(np.prod(shape)) > GRID_STRIDE_ITEMS
+    for tag, amax in (('clamped', 1.3e-8), ('free', 3.7)):
+        a = rand(800, *shape, lo=-0.5 * amax, hi=0.5 * amax)
+        a.view(-1)[-1] = -amax
+        sc = ops.GradScale(DEV).from_amax(a.to(DEV))
+        torch.cuda.synchronize()
+        want = _host_scale(float(np.float32(amax)))
+        out[f'scale_log2_{tag}'] = float(np.log2(float(sc.ws[0])))
+        assert float(sc.ws[0]) == want and float(sc.ws[1]) == 1.0 / want, (tag, float(sc.ws[0]), want)
+        assert (want == 2.0 ** 24) == (tag == 'clamped')
+    # ---- grad_pack (a + b) * scale -> NHWC fp16 and grad_unpack back to NCHW fp32 / scale (accumulating)
+    n, c, h, w = 38, 3, 256, 256
+    a, b = rand(801, n, c, h, w, lo=-1e-8, hi=1e-8), rand(802, n, c, h, w, lo=-1e-8, hi=1e-8)
+    a[-1, -1, -1, -1], b[-1, -1, -1, -1] = 3e-8, 1e-8          # the largest value: last element of the last pass
+    sc = ops.GradScale(DEV).from_amax(a.to(DEV), b.to(DEV))
+    pk = ops.grad_pack(a.to(DEV), b.to(DEV), scale=sc, cpad=64)
+    torch.cuda.synchronize()
+    s = float(sc.ws[0])
+    assert s == _host_scale(max(float(a.abs().max()), float(b.abs().max()))), s
+    want = ((a + b) * s).half()
+    got = pk.cpu()
+    assert torch.equal(got[..., :c], want.permute(0, 2, 3, 1)), 'grad_pack differs from fp16((a + b) * scale)'
+    assert float(got[..., c:].abs().max()) == 0.0, 'grad_pack pad channels must be zero'
+    base = rand(803, n, c, h, w, lo=-1, hi=1)
+    y = base.to(DEV)
+    ops.grad_unpack(pk, c, scale=sc, y=y, accumulate=True)
+    torch.cuda.synchronize()
+    ref = base.double() + want.double() / s
+    out['grad_unpack_max_abs'] = float((y.cpu().double() - ref).abs().max())
+    assert torch.equal(y.cpu(), base + want.float() / s), 'grad_unpack must be exact: fp16 * 2^-k + fp32 in fp32'
+    out['grad_pack_roundtrip_rel_l2'] = rell2((want.double() / s).numpy(), (a.double() + b.double()).numpy())
+    assert out['grad_pack_roundtrip_rel_l2'] <= 1e-3, out          # fp16 rounding of the scaled values
+    del a, b, pk, y, base, want, got
+    # ---- bias gradient over 40x256x256 = 2.6 M pixels (the transposed-conv path), pre-filled db, loss scale
+    npx_n = 40
+    dz = torch.empty(npx_n, 256, 256, 64, dtype=torch.float16).uniform_(-1, 1, generator=torch.Generator().manual_seed(804))
+    dz[-1, -1, -1, 5] = 2000.0                             # decisive value in the very last pixel
+    assert npx_n * 256 * 256 > 2 * GRID_STRIDE_ITEMS
+    sc = ops.GradScale(DEV).from_amax(torch.full((1, 1, 1, 1), 1.5, device=DEV))
+    db = torch.linspace(-1, 1, 64).to(DEV)
+    ops.bias_grad(dz.to(DEV), db, sc)
+    torch.cuda.synchronize()
+    s = float(sc.ws[0])
+    assert s == _host_scale(1.5) == 128.0, s
+    ref = torch.linspace(-1, 1, 64).double() + dz.sum((0, 1, 2), dtype=torch.float64) / s
+    out['bias_grad_rel_l2'] = rell2(db.cpu().numpy(), ref.numpy())
+    out['bias_grad_ch5_rel'] = abs(float(db[5]) - float(ref[5])) / abs(float(ref[5]))
+    assert out['bias_grad_rel_l2'] <= 1e-5 and out['bias_grad_ch5_rel'] <= 1e-5, out
+    del dz
+    # ---- fused warp + s2d + concat backward on 24 HR frames of 256x256 (1.57 M pixels), loss-scaled gx
+    from oracle import frnet_torchref as R
+    n, S, h, w = 24, 4, 64, 64
+    assert n * S * h * S * w > GRID_STRIDE_ITEMS
+    hp = rand(805, n, 3, S * h, S * w)
+    hf = rand(806, n, 2, S * h, S * w, lo=-3, hi=3)
+    hf[-1, :, -1, -1] = torch.tensor([-40.0, -70.0])           # the last pixel samples far across the frame
+    # flows on a 2^-12 grid offset by 2^-13: x + flow is exact in fp32 and never within 2^-13 of a pixel line, where
+    # the flow gradient of bilinear sampling jumps (else the fp32 rounding of the coordinate moves ~1 pixel in 3e4
+    # to the neighbouring cell, an O(1) change that is the conditioning of the operation, not a kernel error)
+    hf = torch.floor(hf * 4096.0) / 4096.0 + 1.0 / 8192.0
+    g = rand(807, n, 51, h, w, lo=-1e-8, hi=1e-8)
+    g[-1, :, -1, -1] *= 50.0
+    sc = ops.GradScale(DEV).from_amax(g.to(DEV))
+    s = float(sc.ws[0])
+    assert s == _host_scale(float(g.abs().max())), s
+    g16 = (g * s).half()
+    hp64 = hp.double().requires_grad_(True)
+    hf64 = hf.double().requires_grad_(True)
+    xx = R.s2d(R.warp(hp64, hf64), S)
+    ghp_ref, ghf_ref = torch.autograd.grad(xx, [hp64, hf64], g16[:, 3:].double() / s)
+    pre = rand(808, n, 3, S * h, S * w, lo=-1e-8, hi=1e-8)
+    d_hp = pre.to(DEV)
+    d_hf = torch.full((n, 2, S * h, S * w), float('nan'), device=DEV)
+    ops.warp_s2d_concat_bwd(nhwc(g16.float()), hp.to(DEV), hf.to(DEV), S, d_hr_prev=d_hp, d_hr_flow=d_hf, scale=sc)
+    torch.cuda.synchronize()
+    got_hp = d_hp.cpu().double() - pre.double()
+    out['fused_warp_dhr_rel_l2'] = rell2(got_hp.numpy(), ghp_ref.numpy())
+    out['fused_warp_dflow_rel_l2'] = rell2(d_hf.cpu().numpy(), ghf_ref.numpy())
+    out['fused_warp_dhr_last_img_rel_l2'] = rell2(got_hp[-1].numpy(), ghp_ref[-1].numpy())
+    assert out['fused_warp_dhr_rel_l2'] <= 1e-4 and out['fused_warp_dhr_last_img_rel_l2'] <= 1e-4, out
+    assert out['fused_warp_dflow_rel_l2'] <= 1e-4, out          # same sample points: the closed form is exact
+    return out
+
+
+# =============================================================================== full-depth BPTT
+def _frvsr_losses(d, gt, warp):
+    """the FRVSR training losses of frvsr_train_step: Charbonnier pixel loss + Charbonnier warping loss"""
+    return _charbonnier(d['hr_data'], gt), _charbonnier(warp(d['lr_prev'], d['lr_flow']), d['lr_curr'])
+
+
+def _record_max(store, key, fn):
+    def wrapped(*args, **kwargs):
+        y = fn(*args, **kwargs)
+        store[key] = max(store.get(key, 0.0), float(y.float().abs().max()))
+        return y
+    return wrapped
+
+
+def check_sequence_grads_full_depth(n=2, t=10, lr=32, seed=41):
+    """The generator backward at full depth: define_generator(FRVSR_OPT) (10 residual blocks, 4x BD), 2 clips of a
+    10-frame ping-pong (19 frames), LR 32x32, the FRVSR losses, forward + backward without the optimizer step, on
+    (a) the GPU, (b) the fp16 CPU precision model (tests/fake_ops.py on a separate FRNet, installed only inside a
+    MonkeyPatch context) and (c) R.forward_sequence in float64.  Bars: every gradient finite; per parameter,
+    rel-L2(a, c) <= 1.5 rel-L2(b, c) + 2e-3 (the pattern of check_step_golden); rel-L2(a, b) <= 1e-2; the logged
+    losses within 1e-3 of (c).  fp16 headroom: the largest |value| PackedDgrad and grad_pack store on the GPU must
+    be finite and <= 2^12 (fp16 max is 65504).  Measured on a B200: rel-L2(a, b) <= 3.0e-3, at most 0.51 of the
+    bar against (c), losses within 1.5e-5, largest stored fp16 gradient 37 (the CPU model's too)."""
+    import pytest
+    from oracle import frnet_torchref as R
+    here = os.path.dirname(os.path.abspath(__file__))
+    if here not in sys.path:
+        sys.path.insert(0, here)
+    import fake_ops
+    P = 'tecogan-pytorch_b200.'
+    autograd, networks, net_utils = (sys.modules[P + m] for m in ('autograd', 'networks', 'net_utils'))
+    p = O.make_frnet_params(seed, gain=1.0)
+    lr_data, gt = bd_training_data(rand(72, n, t, 3, 4 * lr + 8, 4 * lr + 8).to(DEV))
+    lr_data = torch.cat([lr_data, lr_data.flip(1)[:, 1:]], 1)          # ping-pong: 2t - 1 frames
+    gt = torch.cat([gt, gt.flip(1)[:, 1:]], 1)
+    assert tuple(lr_data.shape) == (n, 2 * t - 1, 3, lr, lr)
+    out = {}
+    # (a) the GPU, recording the largest fp16 gradient the dgrad launches and grad_pack store
+    net = T.define_generator(FRVSR_OPT).to(DEV)
+    net.load_state_dict(p, strict=True)
+    net.train()
+    head = {}
+    with pytest.MonkeyPatch.context() as mp:
+        mp.setattr(ops.PackedDgrad, '__call__', _record_max(head, 'dgrad', ops.PackedDgrad.__call__))
+        mp.setattr(ops, 'grad_pack', _record_max(head, 'grad_pack', ops.grad_pack))
+        lp, lw = _frvsr_losses(net(lr_data), gt, T.backward_warp)
+        (lp + lw).backward()
+        torch.cuda.synchronize()
+    log_a = {'l_pix_G': lp.item(), 'l_warp_G': lw.item()}
+    names = [k for k, _ in net.named_parameters()]
+    ga = {k: v.grad.detach().cpu().double() if v.grad is not None else None for k, v in net.named_parameters()}
+    out['fp16_headroom_gpu'] = dict(head)
+    # (b) the fp16 CPU precision model on its own FRNet and CPU tensors
+    lr_cpu, gt_cpu = lr_data.cpu(), gt.cpu()
+    head_b = {}
+    with pytest.MonkeyPatch.context() as mp:
+        fake_ops.install(mp, ops, networks, net_utils, autograd)
+        mp.setattr(fake_ops, 'STORAGE', torch.float16)
+        mp.setattr(autograd, '_ACT_DTYPE', torch.float16)
+        mp.setattr(ops.PackedDgrad, '__call__', _record_max(head_b, 'dgrad', ops.PackedDgrad.__call__))
+        mp.setattr(ops, 'grad_pack', _record_max(head_b, 'grad_pack', ops.grad_pack))
+        net_b = T.FRNet(3, 3, 64, 10, 'BD', 4)
+        net_b.load_state_dict(p, strict=True)
+        net_b.train()
+        lp_b, lw_b = _frvsr_losses(net_b(lr_cpu), gt_cpu, T.backward_warp)
+        (lp_b + lw_b).backward()
+    gb = {k: v.grad.detach().double() for k, v in net_b.named_parameters()}
+    out['fp16_headroom_cpu_model'] = dict(head_b)
+    # (c) float64 through the reference's operators
+    q = {k: v.double().requires_grad_(k in names) for k, v in p.items()}
+    lp_c, lw_c = _frvsr_losses(R.forward_sequence(q, lr_cpu.double(), 4, 'BD', nb=10), gt_cpu.double(), R.warp)
+    gc = dict(zip(names, torch.autograd.grad(lp_c + lw_c, [q[k] for k in names])))
+    log_c = {'l_pix_G': lp_c.item(), 'l_warp_G': lw_c.item()}
+    for k in log_c:
+        out['log_rel_' + k] = abs(log_a[k] - log_c[k]) / abs(log_c[k])
+        assert out['log_rel_' + k] <= 1e-3, out
+    missing = [k for k in names if ga[k] is None or not bool(torch.isfinite(ga[k]).all())]
+    assert not missing, f'missing or non-finite gradients: {missing}'
+    worst_c, worst_b, used = 0.0, 0.0, 0.0
+    for k in names:
+        e_ac, e_bc, e_ab = (rell2(ga[k].numpy(), gc[k].numpy()), rell2(gb[k].numpy(), gc[k].numpy()),
+                            rell2(ga[k].numpy(), gb[k].numpy()))
+        if e_ac > worst_c:
+            worst_c, out['worst_vs_fp64'] = e_ac, (k, e_ac, e_bc)
+        if e_ab > worst_b:
+            worst_b, out['worst_vs_cpu_model'] = e_ab, (k, e_ab)
+        used = max(used, e_ac / (1.5 * e_bc + 2e-3))
+        assert e_ac <= 1.5 * e_bc + 2e-3, (k, e_ac, e_bc, out)
+    out['worst_fraction_of_fp64_bar'] = used
+    assert worst_b <= 1e-2, out
+    h = max(head.values())
+    assert np.isfinite(h) and h <= 2.0 ** 12, out
+    return out
+
+
 CHECKS = {
     'warp_hrflow_s4': lambda: check_warp_hrflow(4),
     'warp_hrflow_s2': lambda: check_warp_hrflow(2, h=9, w=70),
@@ -1315,4 +1817,21 @@ CHECKS = {
     'reference_gan_training_integration': check_reference_gan_training_integration,
     'reference_training_integration_ddp': lambda: check_reference_training_integration(ddp=True),
     'step_vs_oracle_fullsize_g15': lambda: check_step_vs_oracle_fullsize(gain=1.5, frames=2),
+    'wgrad_multitile_srnet_conv': lambda: check_wgrad_multitile('srnet_conv'),
+    'wgrad_multitile_conv_out': lambda: check_wgrad_multitile('conv_out'),
+    'wgrad_multitile_convT_64': lambda: check_wgrad_multitile('convT_64'),
+    'wgrad_multitile_convT_128': lambda: check_wgrad_multitile('convT_128'),
+    'wgrad_multitile_fnet_enc1_0': lambda: check_wgrad_multitile('fnet_enc1_0'),
+    'wgrad_multitile_fnet_dec1_0': lambda: check_wgrad_multitile('fnet_dec1_0'),
+    'wgrad_multitile_fnet_dec1_2': lambda: check_wgrad_multitile('fnet_dec1_2'),
+    'wgrad_multitile_fnet_dec2_0': lambda: check_wgrad_multitile('fnet_dec2_0'),
+    'wgrad_multitile_fnet_flow_2': lambda: check_wgrad_multitile('fnet_flow_2'),
+    'wgrad_multitile_max_ctas_sweep': lambda: check_wgrad_multitile('max_ctas_sweep'),
+    'dgrad_multitile_srnet_halo': lambda: check_dgrad_multitile('srnet_halo'),
+    'dgrad_multitile_conv_out': lambda: check_dgrad_multitile('conv_out'),
+    'dgrad_multitile_convT_256_to_128': lambda: check_dgrad_multitile('convT_256_to_128'),
+    'dgrad_multitile_convT_128_to_64': lambda: check_dgrad_multitile('convT_128_to_64'),
+    'dgrad_multitile_fnet_dec2_0': lambda: check_dgrad_multitile('fnet_dec2_0'),
+    'backward_elementwise_large': check_backward_elementwise_large,
+    'sequence_grads_full_depth': check_sequence_grads_full_depth,
 }
